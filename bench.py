@@ -2,9 +2,11 @@
 """bench.py — throughput of the B200 seed-and-extend hot path (BASELINE.json metric: paired 151 bp
 reads/s) with roofline and the reference CPU path beside it.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload bsw|pipeline]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload bsw|pipeline] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one batch of synthetic reads.  See DESIGN.md §Measurement.
+--dump-outputs DIR (default workload) writes the alignment regions of the timed path as DIR/*.npy, so that two builds
+can be compared output for output on the same seeded inputs (see dump_pipeline_outputs).
 """
 from __future__ import annotations
 import argparse, json, os, subprocess, sys, tempfile, threading, time
@@ -346,6 +348,37 @@ def check_against_reference_dump(regs, ro, dump_path, n_reads):
     return int(len(d_regs))
 
 
+DUMP_SAMPLE_READS = 16384
+DUMP_U64_FIELDS = ("c", "hash")
+
+
+def dump_pipeline_outputs(out_dir, regs, ro, seed=1234):
+    """The regions a caller of the timed path receives, as float64 / float32 .npy files (well under 64 MB):
+    regs_per_read.npy (every read), sample_reads.npy (a fixed, seeded sample of DUMP_SAMPLE_READS reads, ascending) and
+    reg_<field>.npy for every field of every region of the sampled reads, in output order.  64-bit unsigned fields are
+    split into <field>_lo / <field>_hi 32-bit halves so that float64 holds them exactly; padding is left out."""
+    os.makedirs(out_dir, exist_ok=True)
+    n = len(ro) - 1
+    per_read = np.diff(ro)
+    assert per_read.max(initial=0) < 1 << 24
+    np.save(os.path.join(out_dir, "regs_per_read.npy"), per_read.astype(np.float32))
+    sample = np.sort(np.random.default_rng(seed).choice(n, min(n, DUMP_SAMPLE_READS), replace=False))
+    np.save(os.path.join(out_dir, "sample_reads.npy"), sample.astype(np.float64))
+    idx = np.concatenate([np.arange(ro[r], ro[r + 1]) for r in sample]) if len(sample) else np.zeros(0, np.int64)
+    sel = regs[idx]
+    for f in regs.dtype.names:
+        if f.startswith("_"):
+            continue
+        v = sel[f]
+        if f in DUMP_U64_FIELDS:
+            v = v.astype(np.uint64)
+            np.save(os.path.join(out_dir, f"reg_{f}_lo.npy"), (v & np.uint64(0xFFFFFFFF)).astype(np.float64))
+            np.save(os.path.join(out_dir, f"reg_{f}_hi.npy"), (v >> np.uint64(32)).astype(np.float64))
+        else:
+            assert v.dtype.kind == "f" or np.abs(v.astype(np.int64)).max(initial=0) < 1 << 53, f
+            np.save(os.path.join(out_dir, f"reg_{f}.npy"), v.astype(np.float64))
+
+
 def run_pipeline(args, rank, world):
     import torch
     pkg = load_package()
@@ -436,6 +469,12 @@ def run_pipeline(args, rank, world):
         t = torch.tensor([ms_step], device="cuda"); torch.distributed.all_reduce(t, op=torch.distributed.ReduceOp.MAX)
         ms_step = float(t.item())
     value = world * n / (ms_step * 1e-3)
+    if args.dump_outputs and rank == 0:
+        # the timed calls leave their regions on the device (copy_out=False); one more call, same batch and sub-batches, copies them out
+        d_regs, d_ro = ctx.seed_chain_extend_resident(codes, offs, d_codes.data_ptr(), d_offs.data_ptr(), True, return_arrays=True)
+        assert len(d_regs) == n_regs, f"regions of the dumped step ({len(d_regs)}) differ from the last timed step ({n_regs})"
+        dump_pipeline_outputs(args.dump_outputs, d_regs, d_ro)
+        del d_regs, d_ro
     # the stages alone: one more pass of the same batch UNSPLIT, so that every kernel is timed without another sub-batch's
     # kernels beside it (the roofline figures below; the timed steps above run args.sub_batches sub-batches in flight,
     # whose per-stage times are sums over sub-batches and overlap each other)
@@ -1013,7 +1052,13 @@ def main():
     ap.add_argument("--pairs", type=int, default=500_000)
     ap.add_argument("--bsw-jobs", type=int, default=4_000_000)
     ap.add_argument("--sub-batches", type=int, default=4, help="sub-batches in flight per GPU (bm2_set_sub_batches); 1 = unsplit")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the regions of the timed path (default workload) as DIR/*.npy; see dump_pipeline_outputs")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and (args.workload != "pipeline" or args.impl != "ours"):
+        ap.error("--dump-outputs is implemented for --workload pipeline --impl ours")
     rank = int(os.environ.get("RANK", 0)); world = int(os.environ.get("WORLD_SIZE", 1))
     if args.impl == "reference":
         out = (run_reference_pipeline(args, rank, world) if args.workload == "pipeline" else

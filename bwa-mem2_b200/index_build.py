@@ -259,7 +259,14 @@ def make_big_reference(total_bp: int, seed: int = 1, n_contigs: int = 24, repeat
             seqs = torch.where(rc[:, None], (3 - seqs).flip(1), seqs)
             pos = torch.randint(0, total_bp - L - 1, (len(u),), device=device, generator=g)
             idx = pos[:, None] + torch.arange(L, device=device)[None, :]
-            G[idx.reshape(-1)] = seqs.reshape(-1)
+            # copies overlap, and a scatter with repeated indices keeps an arbitrary writer on the GPU: keep the last copy of
+            # each position explicitly, so that the genome (and the bench inputs drawn from it) is the same on every run
+            flat = idx.reshape(-1)
+            order = torch.argsort(flat, stable=True)
+            fs = flat[order]
+            last = torch.ones_like(fs, dtype=torch.bool)
+            last[:-1] = fs[1:] != fs[:-1]
+            G[fs[last]] = seqs.reshape(-1)[order[last]]
     w = np.array([0.8 ** i for i in range(n_contigs)], dtype=np.float64)
     lens = np.maximum((w / w.sum() * total_bp).astype(np.int64), 1000)
     lens[0] += total_bp - lens.sum()

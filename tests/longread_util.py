@@ -1,5 +1,5 @@
-"""Shared helper: a small long-read (-x ont2d) data set, index built by the reference binary."""
-import os, subprocess, tempfile, importlib
+"""Shared helper: a small long-read (-x ont2d) data set, index written by bwa_mem2_b200.index_build (the reference's file format)."""
+import os, tempfile, importlib
 import numpy as np
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -21,15 +21,13 @@ def ont2d_opt(capi):
 
 
 def make_dataset(n3k=10, n8k=3, ref_bp=1_000_000):
-    isa = "avx512bw" if "avx512bw" in open("/proc/cpuinfo").read() else "avx2"
-    refbin = os.path.join(ROOT, "oracle", "_ref", isa, "bwa-mem2")
-    if not os.path.exists(refbin):
-        return None
     synth = importlib.import_module("bwa_mem2_b200.synth")
+    index_build = importlib.import_module("bwa_mem2_b200.index_build")
     work = tempfile.mkdtemp(prefix="bm2_long_")
     ctg = synth.make_reference(ref_bp, seed=9, n_contigs=3)
     synth.write_fasta(work + "/ref.fa", ctg)
-    subprocess.check_call([refbin, "index", work + "/ref.fa"], stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL)
+    rng = np.random.default_rng(10)               # N runs become random bases in the index, as `bwa-mem2 index` does
+    index_build.write_index(work + "/ref.fa", [(n, np.where(c > 3, rng.integers(0, 4, len(c), dtype=np.uint8), c)) for n, c in ctg], device="cpu")
     reads = synth.make_long_reads(ctg, n3k, read_len=3000, seed=4) + synth.make_long_reads(ctg, n8k, read_len=8000, seed=5)
     reads.append(reads[0][:500])          # a short read in the same batch: below the mem_flt_chained_seeds threshold
     codes = np.concatenate(reads); offs = np.concatenate([[0], np.cumsum([len(r) for r in reads])]).astype(np.int64)

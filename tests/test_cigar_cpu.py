@@ -1,11 +1,12 @@
 """Seam 3 (CIGAR / NM / MD == bwa_gen_cigar2, SURVEY 8f item 2) on the CPU: the oracle's restatement against the golden vectors
-made by the UNMODIFIED reference (tests/golden/make_cigar_golden.py) and - when oracle/_ref is built - against the reference
-itself on a fresh random request set; the device logic (cigar_device.cuh compiled for the host) against the oracle."""
-import ctypes as C, os, subprocess
+made by the UNMODIFIED reference (tests/golden/make_cigar_golden.py) and against the reference's results on a second, seeded random
+request set (recorded by tests/golden/make_live_golden.py); the device logic (cigar_device.cuh compiled for the host) against the oracle."""
+import ctypes as C, hashlib, os, subprocess
 import numpy as np
 import pytest
 import oracle_lib as ol
 import cigar_util as cu
+import refgolden
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 _EMUL = None
@@ -65,15 +66,21 @@ def test_device_logic_matches_reference_golden(pkg, c0):
     assert cu.same(got, (g["recs"], g["cigar"], g["md"])) == []
 
 
-def test_oracle_and_device_logic_match_the_live_reference(pkg, c0, golden_dir):
-    if cu.refbin() is None:
-        pytest.skip("oracle/_ref not built")
+def live_requests(capi, idx, codes, offs, read_len):
+    """6000 requests drawn (seeded) from the oracle's regions of the C0 reads, with extra end-point variants."""
+    regs, ro, _, rc = ol.seed_chain_extend(idx, capi.default_opt(), codes, offs)
+    assert rc == 0
+    reqs = cu.make_requests(capi, np.random.default_rng(99), regs, ro, read_len, idx.desc.l_pac, n_extra=1500)
+    return reqs[np.random.default_rng(3).choice(len(reqs), 6000, replace=False)]
+
+
+def test_oracle_and_device_logic_match_the_live_reference(pkg, c0):
     idx, codes, offs, g, read_len = c0
     capi = pkg.capi
-    regs, ro, _, rc = ol.seed_chain_extend(idx, capi.default_opt(), codes, offs)
-    reqs = cu.make_requests(capi, np.random.default_rng(99), regs, ro, read_len, idx.desc.l_pac, n_extra=1500)
-    reqs = reqs[np.random.default_rng(3).choice(len(reqs), 6000, replace=False)]
-    want = cu.reference_gen_cigar(capi, golden_dir + "/c0_index/ref.fa", codes, offs, reqs)
+    reqs = live_requests(capi, idx, codes, offs, read_len)
+    assert hashlib.sha256(reqs.tobytes()).hexdigest() == refgolden.get("cigar/reqs_sha256").tobytes().decode(), \
+        "the request set differs from the one the reference was run on"
+    want = tuple(refgolden.get("cigar/" + k) for k in ("recs", "cigar", "md"))
     got = ol.gen_cigar(idx, capi.default_opt(), codes, offs, reqs)
     assert got[3] == 0 and cu.same(got[:3], want) == []
     assert cu.same(emul_gen_cigar(capi, idx, capi.default_opt(), codes, offs, reqs), want) == []

@@ -13,10 +13,7 @@ def test_long_reads_match_oracle(pkg, coop_min, monkeypatch):
     # coop_min = 0: every read of the warp-per-read pass runs its chaining on all 32 lanes (ChainWarp: ballots for the tree scans, block shifts)
     if coop_min is not None:
         monkeypatch.setenv("BM2_CHAIN_COOP_MIN", coop_min)
-    ds = lu.make_dataset(n3k=10, n8k=3, ref_bp=1_000_000)
-    if ds is None:
-        pytest.skip("oracle/_ref not built")
-    prefix, codes, offs = ds
+    prefix, codes, offs = lu.make_dataset(n3k=10, n8k=3, ref_bp=1_000_000)
     idx = pkg.capi.Index(prefix); opt = lu.ont2d_opt(pkg.capi)
     ctx = pkg.capi.Context(0, index=idx, opt=opt)
     got, go = ctx.seed_chain_extend(codes, offs)

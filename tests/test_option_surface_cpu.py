@@ -1,15 +1,14 @@
 """The mem_opt_t parameter surface of the hot path (`bwa-mem2 mem` options -k -w -A -B -O -E -L -c -d -r -D -s -G -N -W -y -X):
-the UNMODIFIED reference is run with the options on the C0 reads (oracle/_ref/*/ref_driver, regs dumped by the link-time
-hooks), the same options are set in bm2_mem_opt_t the way src/fastmap.cpp does (incl. update_a and bwa_fill_scmat), and both
-the oracle and the kernels' device logic (host emulation) must reproduce every field of every alignment region.
-Needs oracle/_ref (built by __graft_entry__.build() where /root/reference exists; it travels to the GPU box)."""
-import os, subprocess, tempfile
+the regs of the UNMODIFIED reference run with the options on the C0 reads (ref_driver's link-time hooks; recorded by
+tests/golden/make_live_golden.py), the same options are set in bm2_mem_opt_t the way src/fastmap.cpp does (incl. update_a
+and bwa_fill_scmat), and both the oracle and the kernels' device logic (host emulation) must reproduce every field of every
+alignment region."""
+import os, shutil, tempfile
 import numpy as np
 import pytest
 import oracle_lib as ol
 import emul_lib as el
-import refdump
-import cigar_util as cu
+import refgolden
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -88,35 +87,26 @@ def opt_from_cli(capi, args):
     return o
 
 
+# the .alt file of test_alt_contigs: two of the four C0 contigs are ALT contigs of the first
+ALT_FILE = "chr3\t0\tchr1\t1\t60\t100M\t*\t0\t0\t*\t*\nchr4\t0\tchr1\t1\t60\t100M\t*\t0\t0\t*\t*\n"
+
+
 @pytest.fixture(scope="module")
 def c0(pkg, golden_dir):
-    if cu.refbin() is None:
-        pytest.skip("oracle/_ref not built")
     idx = pkg.capi.Index(golden_dir + "/c0_index/ref.fa")
     reads = np.load(golden_dir + "/c0_reads.npz")["reads"]
     codes = reads.reshape(-1); offs = (np.arange(len(reads) + 1) * reads.shape[1]).astype(np.int64)
-    # FASTQ of the C0 reads (pairs interleaved in the fixture)
-    work = tempfile.mkdtemp(prefix="bm2_opt_")
-    for k, name in ((0, "r1.fq"), (1, "r2.fq")):
-        with open(os.path.join(work, name), "w") as f:
-            for i, r in enumerate(reads[k::2]):
-                f.write(f"@p{i}\n{''.join('ACGTN'[c] for c in r)}\n+\n{'I' * len(r)}\n")
-    yield idx, codes, offs, work, golden_dir + "/c0_index/ref.fa"
+    yield idx, codes, offs, golden_dir + "/c0_index/ref.fa"
     idx.close()
 
 
 @pytest.mark.parametrize("name,args", CASES, ids=[c[0] for c in CASES])
 def test_reference_oracle_and_device_logic_agree(pkg, c0, name, args):
-    idx, codes, offs, work, prefix = c0
-    env = dict(os.environ, BM2_DUMP_PREFIX=os.path.join(work, name))
-    with open(os.path.join(work, name + ".sam"), "w") as f:
-        subprocess.check_call([cu.refbin(), "mem", "-t", "1", "-K", "100000000"] + args + [prefix, os.path.join(work, "r1.fq"), os.path.join(work, "r2.fq")],
-                              stdout=f, stderr=subprocess.DEVNULL, env=env)
-    ref_regs, ref_off = refdump.read_regs(os.path.join(work, name + ".regs.bin"))
+    idx, codes, offs, prefix = c0
     opt = opt_from_cli(pkg.capi, args)
     regs, ro, cells, rc = ol.seed_chain_extend(idx, opt, codes, offs)
     assert rc == 0
-    assert ol.regs_equal_to_dump(regs, ro, ref_regs, ref_off) == [], "oracle differs from the reference"
+    assert refgolden.regs_differ(f"opt/{name}", regs, ro) == [], "oracle differs from the reference"
     eregs, ero = el.seed_chain_extend(idx, opt, codes, offs)
     assert np.array_equal(ero, ro) and eregs.tobytes() == regs.tobytes(), "device logic differs from the oracle"
     assert len(regs) > 1000
@@ -124,24 +114,18 @@ def test_reference_oracle_and_device_logic_agree(pkg, c0, name, args):
 
 def test_alt_contigs(pkg, c0, golden_dir):
     """ALT-aware chaining / marking (src/bwamem.cpp:506-624, :1164-1168): the C0 index with a .alt file naming two of its four contigs."""
-    import shutil
-    idx0, codes, offs, work, prefix0 = c0
-    d = os.path.join(work, "altidx"); os.makedirs(d, exist_ok=True)
+    idx0, codes, offs, prefix0 = c0
+    d = tempfile.mkdtemp(prefix="bm2_alt_")
     for f in os.listdir(os.path.dirname(prefix0)):
         shutil.copy(os.path.join(os.path.dirname(prefix0), f), os.path.join(d, f))
     with open(os.path.join(d, "ref.fa.alt"), "w") as f:
-        f.write("chr3\t0\tchr1\t1\t60\t100M\t*\t0\t0\t*\t*\nchr4\t0\tchr1\t1\t60\t100M\t*\t0\t0\t*\t*\n")
+        f.write(ALT_FILE)
     prefix = os.path.join(d, "ref.fa")
-    env = dict(os.environ, BM2_DUMP_PREFIX=os.path.join(work, "alt"))
-    with open(os.path.join(work, "alt.sam"), "w") as f:
-        subprocess.check_call([cu.refbin(), "mem", "-t", "1", "-K", "100000000", prefix, os.path.join(work, "r1.fq"), os.path.join(work, "r2.fq")],
-                              stdout=f, stderr=subprocess.DEVNULL, env=env)
-    ref_regs, ref_off = refdump.read_regs(os.path.join(work, "alt.regs.bin"))
     idx = pkg.capi.Index(prefix)
     opt = pkg.capi.default_opt()
     regs, ro, cells, rc = ol.seed_chain_extend(idx, opt, codes, offs)
-    assert rc == 0 and (ref_regs["is_alt"] != 0).sum() > 1000
-    assert ol.regs_equal_to_dump(regs, ro, ref_regs, ref_off) == []
+    assert rc == 0 and refgolden.regs_differ("opt/alt", regs, ro) == []
+    assert (((regs["n_comp_is_alt"] >> 30) & 3) != 0).sum() > 1000
     eregs, ero = el.seed_chain_extend(idx, opt, codes, offs)
     assert np.array_equal(ero, ro) and eregs.tobytes() == regs.tobytes()
     idx.close()

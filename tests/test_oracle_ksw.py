@@ -1,10 +1,11 @@
 """Mate-rescue local alignment (SURVEY 8f item 1, groundwork for the next widening step): the oracle's scalar restatement of the
 reference's striped SSE2 kernels (ksw_align2 = ksw_u8 / ksw_i16 forward + reversed-prefix pass, src/ksw.cpp:111-381) against
-golden vectors made by the UNMODIFIED reference (tests/golden/make_ksw_golden.py) and, when oracle/_ref is built, against the
-reference itself on fresh request sets."""
+golden vectors made by the UNMODIFIED reference (tests/golden/make_ksw_golden.py) and against the reference's results on seeded request
+sets of other query lengths (recorded by tests/golden/make_live_golden.py)."""
 import numpy as np
 import pytest
 import ksw_util as ku
+import refgolden
 
 
 def _golden(golden_dir):
@@ -21,12 +22,13 @@ def test_oracle_matches_reference_golden(pkg, golden_dir):
     assert sum(1 for r in reqs if r[2] & ku.KSW_XBYTE) > 500 and sum(1 for r in reqs if not r[2] & ku.KSW_XBYTE) > 200      # both kernels
 
 
-@pytest.mark.parametrize("seed,qlens", [(11, (151,)), (12, (36, 50, 76, 100)), (13, (249, 250, 251, 400)), (14, (15, 16, 17, 8, 9))])
+KSW_CASES = [(11, (151,)), (12, (36, 50, 76, 100)), (13, (249, 250, 251, 400)), (14, (15, 16, 17, 8, 9))]
+
+
+@pytest.mark.parametrize("seed,qlens", KSW_CASES)
 def test_oracle_matches_the_live_reference(pkg, seed, qlens):
-    if ku.refbin() is None:
-        pytest.skip("oracle/_ref not built")
     reqs = ku.make_requests(np.random.default_rng(seed), 1200, qlens=qlens)
-    want = ku.reference_ksw(reqs)
+    want = refgolden.get(f"ksw/{seed}")
     got = ku.oracle_ksw(reqs, pkg.capi.default_opt())
     bad = np.nonzero((got != want).any(1))[0]
     assert len(bad) == 0, (bad[:5], got[bad[:5]], want[bad[:5]])

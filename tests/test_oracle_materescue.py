@@ -1,11 +1,12 @@
 """Mate rescue around the local alignment (SURVEY 8f item 1, groundwork): the oracle's mem_pestat and mem_matesw against the UNMODIFIED
 reference - mem_pestat through the link-time hook of ref_driver (dump of a normal `mem` run), mem_matesw through `ref_driver matesw`,
-which runs the rescue block of mem_sam_pe with the reference's own mem_matesw on the pairs of a file.  Needs oracle/_ref."""
-import ctypes as C, os, struct, subprocess, tempfile
+which runs the rescue block of mem_sam_pe with the reference's own mem_matesw on the pairs of a file (mate_input).  Both outputs are
+recorded by tests/golden/make_live_golden.py."""
+import ctypes as C, hashlib, os, struct, subprocess
 import numpy as np
 import pytest
 import oracle_lib as ol
-import cigar_util as cu
+import refgolden
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 FIELDS = ("rb", "re", "qb", "qe", "rid", "score", "truesc", "sub", "alt_sc", "csub", "sub_n", "w", "seedcov", "secondary", "secondary_all", "seedlen0",
@@ -14,8 +15,6 @@ FIELDS = ("rb", "re", "qb", "qe", "rid", "score", "truesc", "sub", "alt_sc", "cs
 
 @pytest.fixture(scope="module")
 def c0(pkg, golden_dir):
-    if cu.refbin() is None:
-        pytest.skip("oracle/_ref not built")
     capi = pkg.capi
     idx = capi.Index(golden_dir + "/c0_index/ref.fa")
     reads = np.load(golden_dir + "/c0_reads.npz")["reads"]
@@ -23,23 +22,26 @@ def c0(pkg, golden_dir):
     opt = capi.default_opt()
     regs, ro, _, rc = ol.seed_chain_extend(idx, opt, codes, offs)
     assert rc == 0
-    work = tempfile.mkdtemp(prefix="bm2_mate_")
-    for k, name in ((0, "r1.fq"), (1, "r2.fq")):
-        with open(os.path.join(work, name), "w") as f:
-            for i, r in enumerate(reads[k::2]):
-                f.write(f"@p{i}\n{''.join('ACGTN'[c] for c in r)}\n+\n{'I' * len(r)}\n")
-    env = dict(os.environ, BM2_DUMP_PREFIX=os.path.join(work, "d"))
-    subprocess.check_call([cu.refbin(), "mem", "-t", "1", "-K", "100000000", golden_dir + "/c0_index/ref.fa", os.path.join(work, "r1.fq"), os.path.join(work, "r2.fq")],
-                          stdout=open(os.path.join(work, "o.sam"), "w"), stderr=subprocess.DEVNULL, env=env)
-    buf = open(os.path.join(work, "d.pestat.bin"), "rb").read()
+    buf = refgolden.get("mate/pestat").tobytes()
     assert len(buf) == 4 + 4 * 28
     pes = [struct.unpack_from("<iiidd", buf, 4 + 28 * d) for d in range(4)]
-    yield capi, idx, opt, reads, regs, ro, pes, work, golden_dir + "/c0_index/ref.fa"
+    yield capi, idx, opt, reads, regs, ro, pes
     idx.close()
 
 
+def mate_input(reads, regs, ro, pes):
+    """The input file of `ref_driver matesw`: the pestat bounds, then per read its codes and its regs."""
+    lh = np.array([v for d in range(4) for v in pes[d][:3]], np.int32)
+    out = [lh.tobytes(), struct.pack("<q", len(reads) // 2)]
+    for r in range(len(reads)):
+        out += [struct.pack("<i", reads.shape[1]), reads[r].tobytes()]
+        a = regs[ro[r]:ro[r + 1]]
+        out += [struct.pack("<i", len(a)), a.tobytes()]
+    return b"".join(out)
+
+
 def test_pestat_matches_reference(c0):
-    capi, idx, opt, reads, regs, ro, pes, work, prefix = c0
+    capi, idx, opt, reads, regs, ro, pes = c0
     lh = np.zeros(12, np.int32); as_ = np.zeros(8, np.float64)
     regs_c = np.ascontiguousarray(regs); ro_c = np.ascontiguousarray(ro, np.int64)
     ol.lib().bm2o_pestat(C.byref(opt), C.c_int64(idx.desc.l_pac), C.c_int32(len(reads)), regs_c.ctypes.data_as(C.c_void_p), ro_c.ctypes.data_as(C.c_void_p),
@@ -53,7 +55,7 @@ def test_pestat_matches_reference(c0):
 
 def test_product_pestat_matches_reference(c0):
     """bm2_pestat of the C ABI (host code of the product, bwa-mem2_b200/csrc/pestat.cpp) against the reference's mem_pestat dump."""
-    capi, idx, opt, reads, regs, ro, pes, work, prefix = c0
+    capi, idx, opt, reads, regs, ro, pes = c0
     got = capi.pestat(opt, idx.desc.l_pac, regs, ro)
     for d in range(4):
         assert (int(got[d]["low"]), int(got[d]["high"]), int(got[d]["failed"])) == pes[d][:3], (d, got, pes)
@@ -66,19 +68,11 @@ def test_product_pestat_matches_reference(c0):
 
 
 def test_matesw_matches_reference(c0):
-    capi, idx, opt, reads, regs, ro, pes, work, prefix = c0
-    n_pairs = len(reads) // 2
+    capi, idx, opt, reads, regs, ro, pes = c0
     lh = np.array([v for d in range(4) for v in pes[d][:3]], np.int32)
-    with open(os.path.join(work, "mate_in.bin"), "wb") as f:
-        f.write(lh.tobytes()); f.write(struct.pack("<q", n_pairs))
-        for p in range(n_pairs):
-            for i in (0, 1):
-                r = 2 * p + i
-                f.write(struct.pack("<i", reads.shape[1])); f.write(reads[r].tobytes())
-                a = regs[ro[r]:ro[r + 1]]
-                f.write(struct.pack("<i", len(a))); f.write(a.tobytes())
-    subprocess.check_call([cu.refbin(), "matesw", prefix, os.path.join(work, "mate_in.bin"), os.path.join(work, "mate_out.bin")], stderr=subprocess.DEVNULL)
-    buf = open(os.path.join(work, "mate_out.bin"), "rb").read()
+    assert hashlib.sha256(mate_input(reads, regs, ro, pes)).hexdigest() == refgolden.get("mate/matesw_in_sha256").tobytes().decode(), \
+        "the regs differ from those the reference was given"
+    buf = refgolden.get("mate/matesw_out").tobytes()
     L = ol.lib()
     pos = 0; n_calls = 0; n_sw = 0; n_added = 0
     cur_pair = -1; a = None
@@ -109,7 +103,7 @@ def test_matesw_matches_reference(c0):
 def test_device_logic_of_the_rescue_block_matches_the_oracle(c0):
     """bwa-mem2_b200/csrc/mate_device.cuh (matesw_d, mate_rescue_pair_d over ksw_device.cuh and the tail's sort_dedup_patch_d), compiled for
     the host, against the oracle's chained mem_matesw calls (pinned to the reference by the test above)."""
-    capi, idx, opt, reads, regs, ro, pes, work, prefix = c0
+    capi, idx, opt, reads, regs, ro, pes = c0
     d = os.path.join(ROOT, "tests", "host_emul")
     so = os.path.join(d, "libmateemul.so")
     srcs = [os.path.join(d, "mate_emul.cpp")] + [os.path.join(ROOT, "bwa-mem2_b200", "csrc", f) for f in ("mate_device.cuh", "ksw_device.cuh", "ext_device.cuh", "chain_device.cuh", "hd.h")]

@@ -1,11 +1,12 @@
 """Paired-end SAM stage of the oracle (groundwork for SURVEY 8f): mate rescue + mem_mark_primary_se + mem_pair + the paired / unpaired MAPQ
-logic of mem_sam_pe + the columns of mem_aln2sam, against the committed SAM of the UNMODIFIED reference (tests/golden/c0.sam) and, when
-oracle/_ref is built, against live runs with options: FLAG, RNAME, POS, MAPQ, CIGAR, RNEXT, PNEXT, TLEN, NM, MD, AS, XS of every line."""
+logic of mem_sam_pe + the columns of mem_aln2sam, against the committed SAM of the UNMODIFIED reference (tests/golden/c0.sam) and
+against its SAM of runs with options (recorded by tests/golden/make_live_golden.py): FLAG, RNAME, POS, MAPQ, CIGAR, RNEXT, PNEXT, TLEN,
+NM, MD, AS, XS of every line."""
 import ctypes as C, os, struct, subprocess, tempfile
 import numpy as np
 import pytest
 import oracle_lib as ol
-import cigar_util as cu
+import refgolden
 
 REC_DT = np.dtype([("read", "<i4"), ("flag", "<i4"), ("rid", "<i4"), ("mapq", "<i4"), ("rnext", "<i4"), ("tlen_valid", "<i4"), ("nm", "<i4"), ("score", "<i4"),
                    ("sub", "<i4"), ("n_cigar", "<i4"), ("n_md", "<i4"), ("_pad", "<i4"), ("pos", "<i8"), ("pnext", "<i8"), ("tlen", "<i8"),
@@ -98,20 +99,15 @@ def test_paired_end_sam_matches_reference_golden(c0, golden_dir):
     assert (flags & 0x2).sum() > 800 and (flags & 0x800).sum() >= 3 and (flags & 0x4).sum() >= 5      # proper pairs, supplementary, unmapped
 
 
-@pytest.mark.parametrize("args", [["-a"], ["-M"], ["-P"], ["-S"], ["-Y", "-T", "40"], ["-U", "9"], ["-5"], ["-q"], ["-5", "-P", "-a"], ["-a", "-M"]],
-                         ids=["all", "no_multi", "no_pairing", "no_rescue", "softclip_T40", "U9", "primary5", "keep_supp_mapq", "primary5_P_a", "all_no_multi"])
-def test_paired_end_sam_matches_the_live_reference(c0, golden_dir, args):
-    if cu.refbin() is None:
-        pytest.skip("oracle/_ref not built")
+# option sets of the paired-end runs: (id, `bwa-mem2 mem` arguments)
+PE_CASES = [("all", ["-a"]), ("no_multi", ["-M"]), ("no_pairing", ["-P"]), ("no_rescue", ["-S"]), ("softclip_T40", ["-Y", "-T", "40"]), ("U9", ["-U", "9"]),
+            ("primary5", ["-5"]), ("keep_supp_mapq", ["-q"]), ("primary5_P_a", ["-5", "-P", "-a"]), ("all_no_multi", ["-a", "-M"])]
+
+
+@pytest.mark.parametrize("name,args", PE_CASES, ids=[c[0] for c in PE_CASES])
+def test_paired_end_sam_matches_the_live_reference(c0, name, args):
     capi, idx, reads, codes, offs, names = c0
-    work = tempfile.mkdtemp(prefix="bm2_pe_")
-    for k, name in ((0, "r1.fq"), (1, "r2.fq")):
-        with open(os.path.join(work, name), "w") as f:
-            for i, r in enumerate(reads[k::2]):
-                f.write(f"@p{i}\n{''.join('ACGTN'[c] for c in r)}\n+\n{'I' * len(r)}\n")
-    with open(os.path.join(work, "o.sam"), "w") as f:
-        subprocess.check_call([cu.refbin(), "mem", "-t", "1", "-K", "100000000"] + args + [golden_dir + "/c0_index/ref.fa", os.path.join(work, "r1.fq"),
-                               os.path.join(work, "r2.fq")], stdout=f, stderr=subprocess.DEVNULL)
+    ref_sam = refgolden.sam_lines("pe/" + name)
     opt = capi.default_opt(); opt.flag |= 0x2
     for fl, bit in (("-a", 0x8), ("-M", 0x10), ("-P", 0x4), ("-S", 0x20), ("-Y", 0x200), ("-5", 0x1800), ("-q", 0x1000)):
         if fl in args: opt.flag |= bit
@@ -120,14 +116,11 @@ def test_paired_end_sam_matches_the_live_reference(c0, golden_dir, args):
     regs, ro, _, rc = ol.seed_chain_extend(idx, opt, codes, offs)
     lh, as_ = _pestat(capi, idx, opt, reads, regs, ro)
     recs, cig, md = oracle_sam_pe(capi, idx, opt, codes, offs, regs, ro, lh, as_)
-    _compare(fields(recs, cig, md, names), parse_sam(open(os.path.join(work, "o.sam"))))
+    _compare(fields(recs, cig, md, names), parse_sam(ref_sam))
     # the device logic's records, formatted by tests/sam_text.py, against the reference's text (from FLAG on)
     import sam_text
     e_recs, e_cig, e_md, e_xa, e_aux = emul_sam_pe(capi, idx, opt, codes, offs, regs, ro, lh, as_, xa_names=names)
-    want = [ln.rstrip("\n").split("\t", 1)[1] for ln in open(os.path.join(work, "o.sam")) if not ln.startswith("@")]
-    got = sam_text.format_lines(e_recs, e_cig, e_md, e_xa, names, codes, offs, is_alt=e_aux[:, 1], n_mc=e_aux[:, 2])
-    bad = [i for i in range(len(want)) if got[i] != want[i]]
-    assert len(got) == len(want) and not bad, (len(bad), [(got[i], want[i]) for i in bad[:2]])
+    refgolden.assert_sam_text("pe/" + name, sam_text.format_lines(e_recs, e_cig, e_md, e_xa, names, codes, offs, is_alt=e_aux[:, 1], n_mc=e_aux[:, 2]))
 
 
 def oracle_sam_text(capi, idx, opt, codes, offs, regs, ro, lh, as_, names, qual_char="I"):
@@ -161,13 +154,13 @@ def test_paired_end_sam_text_is_byte_identical_to_the_reference_golden(c0, golde
     assert sum("SA:Z:" in w for w in want) >= 6 and sum("MC:Z:" in w for w in want) > 900
 
 
-def test_sam_text_with_xa_and_alt_tags_matches_the_live_reference(pkg):
-    """A genome with 2-4 copy segmental duplications (XA tags) and ALT contigs (pa tag, ALT-aware primary marking): byte-identical text."""
-    if cu.refbin() is None:
-        pytest.skip("oracle/_ref not built")
-    capi = pkg.capi
+XA_ALT = "c1_alt\t0\tc1\t20001\t60\t40000M\t*\t0\t0\t*\t*\n"
+
+
+def xa_dataset(work):
+    """A genome with 2-4 copy segmental duplications and an ALT contig, written to work/ref.fa (+ .alt), and 1500 read pairs written to
+    work/r1.fq, work/r2.fq.  -> (contig names, contigs as 2-bit codes, reads with the pairs interleaved)."""
     rng = np.random.default_rng(12)
-    work = tempfile.mkdtemp(prefix="bm2_xa_")
     ctgs = []
     for c in range(3):
         g = rng.integers(0, 4, 120_000).astype(np.uint8)
@@ -185,10 +178,7 @@ def test_sam_text_with_xa_and_alt_tags_matches_the_live_reference(pkg):
             f.write(f">{n}\n"); s = "".join("ACGT"[b] for b in g)
             f.write("\n".join(s[i:i + 80] for i in range(0, len(s), 80)) + "\n")
     with open(work + "/ref.fa.alt", "w") as f:
-        f.write("c1_alt\t0\tc1\t20001\t60\t40000M\t*\t0\t0\t*\t*\n")
-    bindir = os.path.dirname(cu.refbin())
-    subprocess.check_call([bindir + "/bwa-mem2", "index", work + "/ref.fa"], stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL)
-    genome = np.concatenate(ctgs[:3])
+        f.write(XA_ALT)
     n_pairs = 1500; L = 151
     reads = np.zeros((2 * n_pairs, L), np.uint8)
     comp = np.array([3, 2, 1, 0, 4], np.uint8)
@@ -204,27 +194,32 @@ def test_sam_text_with_xa_and_alt_tags_matches_the_live_reference(pkg):
         with open(os.path.join(work, name), "w") as f:
             for i, r in enumerate(reads[k::2]):
                 f.write(f"@p{i}\n{''.join('ACGTN'[c] for c in r)}\n+\n{'I' * L}\n")
-    env = dict(os.environ, BM2_DUMP_PREFIX=os.path.join(work, "d"))
-    with open(os.path.join(work, "o.sam"), "w") as f:
-        subprocess.check_call([cu.refbin(), "mem", "-t", "1", "-K", "100000000", work + "/ref.fa", work + "/r1.fq", work + "/r2.fq"], stdout=f, stderr=subprocess.DEVNULL, env=env)
-    want = [ln.rstrip("\n").split("\t", 1)[1] for ln in open(work + "/o.sam") if not ln.startswith("@")]
+    return names, ctgs, reads
+
+
+def test_sam_text_with_xa_and_alt_tags_matches_the_live_reference(pkg):
+    """A genome with 2-4 copy segmental duplications (XA tags) and ALT contigs (pa tag, ALT-aware primary marking): byte-identical text
+    against the reference's SAM of the same reads on the same genome (its index written by bwa_mem2_b200.index_build, which writes the
+    reference's index bytes)."""
+    import importlib
+    capi = pkg.capi
+    work = tempfile.mkdtemp(prefix="bm2_xa_")
+    names, ctgs, reads = xa_dataset(work)
+    importlib.import_module("bwa_mem2_b200.index_build").write_index(work + "/ref.fa", list(zip(names, ctgs)), device="cpu")
+    L = reads.shape[1]
+    want = [ln.rstrip("\n").split("\t", 1)[1] for ln in refgolden.sam_lines("pe/xa_alt")]
     idx = capi.Index(work + "/ref.fa")
     opt = capi.default_opt(); opt.flag |= 0x2
     codes = reads.reshape(-1); offs = (np.arange(len(reads) + 1) * L).astype(np.int64)
     regs, ro, _, rc = ol.seed_chain_extend(idx, opt, codes, offs)
     lh, as_ = _pestat(capi, idx, opt, reads, regs, ro)
-    got = oracle_sam_text(capi, idx, opt, codes, offs, regs, ro, lh, as_, names)
-    assert len(got) == len(want)
-    bad = [i for i in range(len(got)) if got[i] != want[i]]
-    assert not bad, (len(bad), [(got[i], want[i]) for i in bad[:2]])
+    refgolden.assert_sam_text("pe/xa_alt", oracle_sam_text(capi, idx, opt, codes, offs, regs, ro, lh, as_, names))
     assert sum("XA:Z:" in w for w in want) > 30 and sum("pa:f:" in w for w in want) > 5, (sum("XA:Z:" in w for w in want), sum("pa:f:" in w for w in want))
     # the device logic's XA entries (sam_gen_alt_d) against the reference's XA tags, record by record
     e_recs, e_cig, e_md, e_xa, e_aux = emul_sam_pe(capi, idx, opt, codes, offs, regs, ro, lh, as_, xa_names=names)
     assert e_xa == xa_of_lines(want)
     import sam_text                                                  # ... and the whole text from the records: SEQ / QUAL, MC, SA, pa included
-    txt = sam_text.format_lines(e_recs, e_cig, e_md, e_xa, names, codes, offs, is_alt=e_aux[:, 1], n_mc=e_aux[:, 2])
-    bad = [i for i in range(len(want)) if txt[i] != want[i]]
-    assert not bad, (len(bad), [(txt[i], want[i]) for i in bad[:2]])
+    refgolden.assert_sam_text("pe/xa_alt", sam_text.format_lines(e_recs, e_cig, e_md, e_xa, names, codes, offs, is_alt=e_aux[:, 1], n_mc=e_aux[:, 2]))
     pa_want = [([f for f in w.split("\t") if f.startswith("pa:f:")] or [""])[0] for w in want]
     pa_got = [("pa:f:%.3f" % (float(r["score"]) / float(r["_pad"]))) if r["_pad"] > 0 and not (r["flag"] & 0x100) else "" for r in e_recs]
     assert pa_got == pa_want                                         # SamRec::alt_sc

@@ -1,11 +1,12 @@
 """Single-end SAM stage of the oracle (groundwork for SURVEY 8f items 2-3): mem_mark_primary_se, mem_approx_mapq_se, mem_reg2aln and the
-record selection of mem_reg2sam against the SAM the UNMODIFIED reference writes for the same reads in single-end mode
-(FLAG, RNAME, POS, MAPQ, CIGAR with soft / hard clips, NM, MD, AS, XS of every line, supplementary lines included).  Needs oracle/_ref."""
-import ctypes as C, os, subprocess, tempfile
+record selection of mem_reg2sam against the SAM the UNMODIFIED reference writes for the same reads in single-end mode (recorded by
+tests/golden/make_live_golden.py): FLAG, RNAME, POS, MAPQ, CIGAR with soft / hard clips, NM, MD, AS, XS of every line, supplementary
+lines included."""
+import ctypes as C
 import numpy as np
 import pytest
 import oracle_lib as ol
-import cigar_util as cu
+import refgolden
 
 ALN_DT = np.dtype([("read", "<i4"), ("flag", "<i4"), ("rid", "<i4"), ("mapq", "<i4"), ("nm", "<i4"), ("score", "<i4"), ("sub", "<i4"), ("is_rev", "<i4"),
                    ("is_alt", "<i4"), ("alt_sc", "<i4"), ("n_cigar", "<i4"), ("n_md", "<i4"), ("pos", "<i8"), ("cigar_off", "<i8"), ("md_off", "<i8")])
@@ -53,9 +54,9 @@ def sam_fields(alns, cigar, md, names, soft_clip_all=False):
     return lines
 
 
-def parse_sam(path):
+def parse_sam(lines):
     out = []
-    for ln in open(path):
+    for ln in lines:
         if ln.startswith("@"):
             continue
         f = ln.rstrip("\n").split("\t")
@@ -67,22 +68,21 @@ def parse_sam(path):
     return out
 
 
-@pytest.mark.parametrize("args", [[], ["-a"], ["-M"], ["-T", "50"], ["-Y"], ["-5"], ["-q"]], ids=["default", "all", "no_multi", "T50", "softclip", "primary5", "keep_supp_mapq"])
-def test_single_end_sam_matches_reference(pkg, golden_dir, args):
-    if cu.refbin() is None:
-        pytest.skip("oracle/_ref not built")
+# option sets of the single-end runs (the reads of the r1 file of C0): (id, `bwa-mem2 mem` arguments)
+SE_CASES = [("default", []), ("all", ["-a"]), ("no_multi", ["-M"]), ("T50", ["-T", "50"]), ("softclip", ["-Y"]), ("primary5", ["-5"]), ("keep_supp_mapq", ["-q"])]
+
+
+def se_reads(golden_dir):
+    return np.load(golden_dir + "/c0_reads.npz")["reads"][0::2]              # the r1 file
+
+
+@pytest.mark.parametrize("name,args", SE_CASES, ids=[c[0] for c in SE_CASES])
+def test_single_end_sam_matches_reference(pkg, golden_dir, name, args):
     capi = pkg.capi
     idx = capi.Index(golden_dir + "/c0_index/ref.fa")
-    reads = np.load(golden_dir + "/c0_reads.npz")["reads"][0::2]            # the r1 file
+    reads = se_reads(golden_dir)
     codes = reads.reshape(-1); offs = (np.arange(len(reads) + 1) * reads.shape[1]).astype(np.int64)
-    work = tempfile.mkdtemp(prefix="bm2_se_")
-    with open(os.path.join(work, "r1.fq"), "w") as f:
-        for i, r in enumerate(reads):
-            f.write(f"@p{i}\n{''.join('ACGTN'[c] for c in r)}\n+\n{'I' * len(r)}\n")
-    with open(os.path.join(work, "o.sam"), "w") as f:
-        subprocess.check_call([cu.refbin(), "mem", "-t", "1", "-K", "100000000"] + args + [golden_dir + "/c0_index/ref.fa", os.path.join(work, "r1.fq")],
-                              stdout=f, stderr=subprocess.DEVNULL)
-    want = parse_sam(os.path.join(work, "o.sam"))
+    want = parse_sam(refgolden.sam_lines("se/" + name))
     opt = capi.default_opt()
     if "-a" in args: opt.flag |= 0x8
     if "-M" in args: opt.flag |= 0x10
@@ -134,22 +134,13 @@ def rec_fields(recs, cigar, md, names):
     return out
 
 
-@pytest.mark.parametrize("args", [[], ["-a"], ["-M"], ["-T", "50"], ["-Y"], ["-5"]], ids=["default", "all", "no_multi", "T50", "softclip", "primary5"])
-def test_single_end_device_logic_matches_reference(pkg, golden_dir, args):
-    if cu.refbin() is None:
-        pytest.skip("oracle/_ref not built")
+@pytest.mark.parametrize("name,args", SE_CASES[:6], ids=[c[0] for c in SE_CASES[:6]])
+def test_single_end_device_logic_matches_reference(pkg, golden_dir, name, args):
     capi = pkg.capi
     idx = capi.Index(golden_dir + "/c0_index/ref.fa")
-    reads = np.load(golden_dir + "/c0_reads.npz")["reads"][0::2]
+    reads = se_reads(golden_dir)
     codes = reads.reshape(-1); offs = (np.arange(len(reads) + 1) * reads.shape[1]).astype(np.int64)
-    work = tempfile.mkdtemp(prefix="bm2_se_")
-    with open(os.path.join(work, "r1.fq"), "w") as f:
-        for i, r in enumerate(reads):
-            f.write(f"@p{i}\n{''.join('ACGTN'[c] for c in r)}\n+\n{'I' * len(r)}\n")
-    with open(os.path.join(work, "o.sam"), "w") as f:
-        subprocess.check_call([cu.refbin(), "mem", "-t", "1", "-K", "100000000"] + args + [golden_dir + "/c0_index/ref.fa", os.path.join(work, "r1.fq")],
-                              stdout=f, stderr=subprocess.DEVNULL)
-    want = parse_sam(os.path.join(work, "o.sam"))
+    want = parse_sam(refgolden.sam_lines("se/" + name))
     opt = capi.default_opt()
     if "-a" in args: opt.flag |= 0x8
     if "-M" in args: opt.flag |= 0x10
